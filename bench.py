@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- correspondence + linearisation + reduction throughput of the small_gicp hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--points P] [--no-extras]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--points P] [--no-extras] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 Headline workload (BASELINE.json configs[1]): synthetic room pair, P = 1,000,000 target points and 1,000,000 source points PER GPU,
@@ -23,6 +23,9 @@ Extras on the same line (the other BASELINE configs on hardware; skipped with --
 `c5`           configs[4]: linearize over 100k .. 100M points (ONE cloud pair, source strong-sharded over the N GPUs).
 `allreduce_check_rel`  N > 1: |fused sum - NCCL sum of the per-rank local sums| / |sum| (must be <= 1e-12).
 `comm_wait_us` N > 1: time the finishing CTA waited for its peers per exchange: min over ranks = transport, max - min = skew.
+
+--dump-outputs DIR writes what the last timed step returned -- H (6x6), b (6), e and, for our arm, the inlier count -- as float64
+DIR/<name>.npy, so that two builds run with the same arguments (same seeded inputs) can be compared output for output.
 """
 import argparse
 import json
@@ -58,7 +61,18 @@ def parse_args():
     ap.add_argument("--c4-points", type=int, default=10_000_000)
     ap.add_argument("--c3-frames", type=int, default=12)
     ap.add_argument("--leaf", type=int, default=0, help="max leaf size of the device kd-tree (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's H, b, e (and inlier count) as float64 DIR/<name>.npy")
     return ap.parse_args()
+
+
+def dump_outputs(path, H, b, e, num_inliers=None):
+    """--dump-outputs: the sums one linearize hands its caller, float64, one .npy per array"""
+    os.makedirs(path, exist_ok=True)
+    arrays = {"H": np.asarray(H).reshape(6, 6), "b": np.asarray(b).reshape(6), "e": np.asarray([e]).reshape(1)}
+    if num_inliers is not None:
+        arrays["num_inliers"] = np.asarray([num_inliers]).reshape(1)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def dist_env():
@@ -346,8 +360,10 @@ def run_reference(args):
         reg.linearize(tc, tt, sc, poses[i % len(poses)])
     t0 = time.perf_counter()
     for i in range(args.steps):
-        reg.linearize(tc, tt, sc, poses[i % len(poses)])
+        last = reg.linearize(tc, tt, sc, poses[i % len(poses)])
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last)
     ms = dt / args.steps * 1e3
     value = args.points / (ms * 1e-3) / 1e6
     rot, trans = pose_error(inp["T_gt"], T_final)
@@ -921,6 +937,9 @@ def run_ours(args):
             dist.all_reduce(out[:44])
         ev[i][1].record(stream)
     barrier()
+    if args.dump_outputs and rank == 0:  # out holds the last timed step's H|b|e|inliers (all-reduced over the ranks)
+        h = out[:44].cpu().numpy()
+        dump_outputs(args.dump_outputs, h[:36], h[36:42], h[42], h[43])
     launches = ctx.kernel_launches - launches0
     step_ms = np.array([a.elapsed_time(b) for a, b in ev])
     kern_ms = np.array([a.elapsed_time(b) for a, b in kev])

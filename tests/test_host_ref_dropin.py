@@ -3,8 +3,9 @@ tests/host_ref/Makefile) with `Reduction = ParallelReductionCUDA` from include/s
 file INTEGRATION.md tells a maintainer to add -- against the same template on the reference's `ParallelReductionOMP`
 (registration/registration.hpp:31-43, reduction.hpp:20-27,55-56, optimizer.hpp:24-63,83-149).
 
-CPU (`-m "not gpu"`): the harness loads, its OMP arm equals the oracle, the CUDA arm refuses to run without a device (no fallback),
-INTEGRATION.md shows the compiled file verbatim.  GPU (`-m gpu`): same RegistrationResult from both reductions -- pose within
+The harness (oracle/_ref/libsgb_host_ref.so) can only be built where the reference's sources are present; the tests that call it
+skip elsewhere.  CPU (`-m "not gpu"`): the OMP arm's stored results equal the oracle, the CUDA arm refuses to run without a device
+(no fallback), INTEGRATION.md shows the compiled file verbatim.  GPU (`-m gpu`): same RegistrationResult from both reductions -- pose within
 1e-4 rad / 1e-3 m, same `iterations`, `num_inliers` +- 2 -- for every factor x robust kernel x optimizer, VGICP, a source edited in
 place between two align() calls (no stale device mirror), and the generation-counted reuse of the mirror."""
 import ctypes as C
@@ -16,13 +17,13 @@ import pytest
 import oracle as O
 from conftest import ROOT, noise_poses, pose_error
 
-LIB = os.path.join(ROOT, "tests", "host_ref", "libsgb_host_ref.so")
+LIB = os.path.join(ROOT, "oracle", "_ref", "libsgb_host_ref.so")
 _dp = C.POINTER(C.c_double)
 
 
 def _lib():
     if not os.path.exists(LIB):
-        pytest.skip("tests/host_ref/libsgb_host_ref.so not built (needs /root/reference: `make -C tests/host_ref`)")
+        pytest.skip("oracle/_ref/libsgb_host_ref.so not built (it compiles the reference's headers: `make -C tests/host_ref REF=<reference checkout>`)")
     L = C.CDLL(LIB)
     L.href_align.restype = C.c_int
     L.href_align.argtypes = [_dp, C.c_size_t, _dp, _dp, _dp, C.c_size_t, _dp, _dp, _dp, _dp]
@@ -71,16 +72,19 @@ def same_result(r, ref, tag):
 
 # ---------------------------------------------------------------- CPU
 def test_reference_arm_equals_oracle(golden_prepared):
-    """the harness' OMP arm IS the reference (its Registration<> on its ParallelReductionOMP): it must agree with the oracle"""
-    g = golden_prepared
-    for factor, optimizer in ((0, 1), (2, 0), (2, 1)):
+    """the harness' OMP arm IS the reference (its Registration<> on its ParallelReductionOMP): it must agree with the oracle.
+    Its results are stored in tests/golden/reference_outputs.npz (tests/reference_outputs.py), so this runs without the harness."""
+    import reference_outputs as R
+
+    g, stored = golden_prepared, R.load()
+    for factor, optimizer in R.DROPIN_CASES:
         reg = O.Registration(factor=factor, num_threads=0)
         reg.set_optimizer(type=optimizer)
-        for Tn in noise_poses()[:2]:
+        key = f"dropin_omp/{factor}/{optimizer}"
+        for Tn, T_omp, (iterations, num_inliers) in zip(noise_poses()[:2], stored[key + "/T"], stored[key + "/stats"]):
             ref = reg.align(g["target"], g["target_tree"], g["source"], Tn)
-            r = align(OMP, g["target"], g["source"], Tn, factor=factor, optimizer=optimizer)
-            rot, trans = pose_error(ref.T_target_source, r.T_target_source)
-            assert rot < 1e-9 and trans < 1e-9 and r.iterations == ref.iterations and r.num_inliers == ref.num_inliers
+            rot, trans = pose_error(ref.T_target_source, T_omp)
+            assert rot < 1e-9 and trans < 1e-9 and iterations == ref.iterations and num_inliers == ref.num_inliers
 
 
 def test_cuda_arm_has_no_fallback(golden_prepared):

@@ -1,141 +1,90 @@
-"""Pins the oracle's restatement (oracle/sgicp_oracle.cpp) against the REFERENCE'S OWN CODE: oracle/_ref/libsmallgicp_ref.so is
-/root/reference/include compiled in place against the Eigen API shim (oracle/ref_build) behind the same C API.
-Same inputs -> same outputs: bit-exact for integer / index / structure work, <= 1e-12 relative for floating point (the two differ only
-in summation order inside small fixed-size products).  Skipped where the library has not been built (it needs /root/reference)."""
+"""Pins the oracle's restatement (oracle/sgicp_oracle.cpp) against the REFERENCE'S OWN CODE: the outputs of small_gicp's headers
+compiled against the Eigen API shim (oracle/ref_build) on the fixtures of tests/golden, stored in tests/golden/reference_outputs.npz
+by tests/reference_outputs.py.
+Same inputs -> same outputs: bit-exact for integer / index / structure work (compared through SHA-256 digests of the exact bytes),
+<= 1e-12 relative for floating point (the two differ only in summation order inside small fixed-size products); large floating-point
+outputs are compared on a fixed seeded sample of their rows."""
 import numpy as np
 import pytest
 
 import oracle as O
-from conftest import noise_poses
-
-REF = O.reference_lib()
-pytestmark = pytest.mark.skipif(REF is None, reason="oracle/_ref not built (needs /root/reference)")
+import reference_outputs as R
 
 
-def both_clouds(xyz, leaf):
-    a = O.Cloud(xyz).voxelgrid_sampling(leaf)
-    b = O.Cloud(xyz, _lib=REF).voxelgrid_sampling(leaf)
-    return a, b
+@pytest.fixture(scope="module")
+def ref():
+    return R.load()
 
 
 @pytest.fixture(scope="module")
 def prepared(golden):
-    tgt, src, T = golden
-    out = {}
-    for name, lib in (("orc", None), ("ref", REF)):
-        tc = O.Cloud(tgt, _lib=lib).voxelgrid_sampling(0.3)
-        sc = O.Cloud(src, _lib=lib).voxelgrid_sampling(0.3)
-        tt, st = O.KdTree(tc), O.KdTree(sc)
-        tt.estimate(20, O.FEAT_NORMAL_COV, 1)
-        st.estimate(20, O.FEAT_NORMAL_COV, 1)
-        out[name] = (tc, tt, sc, st)
-    out["T"] = T
-    return out
+    return R.prepare(None, golden)
 
 
-@pytest.mark.parametrize("leaf", [0.1, 0.25, 0.3, 1.0])
-def test_voxelgrid_bit_exact(golden, leaf):
-    for xyz in golden[:2]:
-        a, b = both_clouds(xyz, leaf)
-        assert np.array_equal(a.points, b.points)
+def same_digests(out, ref):
+    for k, v in out.items():
+        assert np.array_equal(v, ref[k]), k
 
 
-def test_kdtree_structure_and_knn_bit_exact(prepared):
-    (tc, tt, sc, _), (rc, rt, rsc, _) = prepared["orc"], prepared["ref"]
-    n1, i1 = tt.export()
-    n2, i2 = rt.export()
-    assert np.array_equal(i1, i2)
-    leaf1 = n1.view(np.uint32).reshape(-1, 6)[:, 4] == 0xFFFFFFFF  # left == INVALID_NODE
-    assert np.array_equal(n1.view(np.uint32).reshape(-1, 6)[:, 4:], n2.view(np.uint32).reshape(-1, 6)[:, 4:])
-    # payload: leaves (first,last) 8 bytes; inner nodes axis (4 bytes) + threshold (8 bytes at offset 8); padding bytes are unspecified
-    a, b = n1.view(np.uint32).reshape(-1, 6), n2.view(np.uint32).reshape(-1, 6)
-    assert np.array_equal(a[leaf1, :2], b[leaf1, :2])
-    assert np.array_equal(a[~leaf1, 0], b[~leaf1, 0]) and np.array_equal(a[~leaf1, 2:4], b[~leaf1, 2:4])
-    q = sc.points
-    for k in (1, 5, 20):
-        ia, da, ca = tt.knn(q, k)
-        ib, db, cb = rt.knn(q, k)
-        assert np.array_equal(ia, ib) and np.array_equal(da, db) and np.array_equal(ca, cb)
+@pytest.mark.parametrize("leaf", R.LEAVES)
+def test_voxelgrid_bit_exact(golden, ref, leaf):
+    same_digests(R.voxelgrid_outputs(None, golden, leaf), ref)
 
 
-def test_features_match(prepared):
-    (tc, *_), (rc, *_) = prepared["orc"], prepared["ref"]
-    np.testing.assert_allclose(tc.normals, rc.normals, rtol=0, atol=1e-12)
-    np.testing.assert_allclose(tc.covs, rc.covs, rtol=0, atol=1e-12)
+def test_kdtree_structure_and_knn_bit_exact(prepared, ref):
+    same_digests(R.kdtree_outputs(prepared), ref)
 
 
-CASES = [(f, r) for f in (0, 1, 2) for r in (0, 1, 2)]
+def test_features_match(prepared, ref):
+    out = R.features_outputs(prepared)
+    assert np.array_equal(out["features/rows"], ref["features/rows"])
+    np.testing.assert_allclose(out["features/normals"], ref["features/normals"], rtol=0, atol=1e-12)
+    np.testing.assert_allclose(out["features/covs"], ref["features/covs"], rtol=0, atol=1e-12)
 
 
-@pytest.mark.parametrize("factor,robust", CASES)
-@pytest.mark.parametrize("threads", [0, 2])
-def test_linearize_error_match(prepared, factor, robust, threads):
-    (tc, tt, sc, _), (rc, rt, rsc, _) = prepared["orc"], prepared["ref"]
-    a = O.Registration(factor=factor, robust=robust, robust_c=0.7, num_threads=threads)
-    b = O.Registration(factor=factor, robust=robust, robust_c=0.7, num_threads=threads, _lib=REF)
-    for T in [np.eye(4), prepared["T"]] + noise_poses()[1:2]:
-        Ha, ba, ea = a.linearize(tc, tt, sc, T)
-        Hb, bb, eb = b.linearize(rc, rt, rsc, T)
-        assert np.array_equal(a.correspondences(len(sc)), b.correspondences(len(rsc)))
-        assert np.linalg.norm(Ha - Hb) <= 1e-12 * np.linalg.norm(Hb)
-        assert np.abs(ba - bb).max() <= 1e-11 * np.sqrt(2 * eb * np.diag(Hb)).max()
-        assert abs(ea - eb) <= 1e-12 * eb
-        T2 = T @ O.se3_exp(np.array([0.01, -0.02, 0.005, 0.05, -0.03, 0.02]))
-        e1, e2 = a.error(tc, sc, T2), b.error(rc, rsc, T2)
-        assert abs(e1 - e2) <= 1e-12 * e2
+@pytest.mark.parametrize("factor,robust", R.CASES)
+@pytest.mark.parametrize("threads", R.THREADS)
+def test_linearize_error_match(prepared, golden, ref, factor, robust, threads):
+    out = R.linearize_outputs(None, prepared, golden[2], factor, robust, threads)
+    key = f"linearize/{factor}/{robust}/{threads}"
+    assert np.array_equal(out[key + "/corr"], ref[key + "/corr"])
+    Ha, ba, ea, e1 = (out[key + s] for s in ("/H", "/b", "/e", "/error"))
+    Hb, bb, eb, e2 = (ref[key + s] for s in ("/H", "/b", "/e", "/error"))
+    for j in range(len(eb)):  # identity, ground truth, one noise pose
+        assert np.linalg.norm(Ha[j] - Hb[j]) <= 1e-12 * np.linalg.norm(Hb[j])
+        assert np.abs(ba[j] - bb[j]).max() <= 1e-11 * np.sqrt(2 * eb[j] * np.diag(Hb[j])).max()
+        assert abs(ea[j] - eb[j]) <= 1e-12 * eb[j]
+        assert abs(e1[j] - e2[j]) <= 1e-12 * e2[j]
 
 
-@pytest.mark.parametrize("factor,robust", [(0, 0), (1, 0), (2, 0), (2, 1), (2, 2)])
-@pytest.mark.parametrize("opt", [0, 1])
-def test_align_match(prepared, factor, robust, opt):
-    (tc, tt, sc, _), (rc, rt, rsc, _) = prepared["orc"], prepared["ref"]
-    a = O.Registration(factor=factor, robust=robust, num_threads=0)
-    b = O.Registration(factor=factor, robust=robust, num_threads=0, _lib=REF)
-    a.set_optimizer(type=opt)
-    b.set_optimizer(type=opt)
-    for Tn in noise_poses()[:3]:
-        ra = a.align(tc, tt, sc, Tn)
-        rb = b.align(rc, rt, rsc, Tn)
-        assert ra.iterations == rb.iterations and ra.converged == rb.converged and ra.num_inliers == rb.num_inliers
-        np.testing.assert_allclose(ra.T_target_source, rb.T_target_source, rtol=0, atol=1e-9)
-        assert abs(ra.error - rb.error) <= 1e-9 * max(rb.error, 1e-12)
-        assert np.linalg.norm(ra.H - rb.H) <= 1e-9 * np.linalg.norm(rb.H)
+@pytest.mark.parametrize("factor,robust", R.ALIGN_CASES)
+@pytest.mark.parametrize("opt", R.OPTIMIZERS)
+def test_align_match(prepared, ref, factor, robust, opt):
+    out = R.align_outputs(None, prepared, factor, robust, opt)
+    key = f"align/{factor}/{robust}/{opt}"
+    assert np.array_equal(out[key + "/stats"], ref[key + "/stats"])  # iterations, converged, num_inliers
+    Ta, ea, Ha = (out[key + s] for s in ("/T", "/error", "/H"))
+    Tb, eb, Hb = (ref[key + s] for s in ("/T", "/error", "/H"))
+    for j in range(len(eb)):  # the first three noise poses
+        np.testing.assert_allclose(Ta[j], Tb[j], rtol=0, atol=1e-9)
+        assert abs(ea[j] - eb[j]) <= 1e-9 * max(eb[j], 1e-12)
+        assert np.linalg.norm(Ha[j] - Hb[j]) <= 1e-9 * np.linalg.norm(Hb[j])
 
 
-def test_voxelmap_and_vgicp_match(prepared):
-    (tc, tt, sc, _), (rc, rt, rsc, _) = prepared["orc"], prepared["ref"]
-    for offsets in (1, 7, 27):
-        va, vb = O.GaussianVoxelMap(tc, 1.0, offsets), O.GaussianVoxelMap(rc, 1.0, offsets)
-        ca, ma, cva, na = va.export()
-        cb, mb, cvb, nb = vb.export()
-        assert np.array_equal(ca, cb) and np.array_equal(na, nb)
-        np.testing.assert_allclose(ma, mb, rtol=0, atol=1e-12)
-        np.testing.assert_allclose(cva, cvb, rtol=0, atol=1e-12)
-        ia, da, fa = va.nn(sc.points)
-        ib, db, fb = vb.nn(rsc.points)
-        assert np.array_equal(ia, ib) and np.array_equal(fa, fb)
-        np.testing.assert_allclose(da[fa == 1], db[fb == 1], rtol=1e-12)
-        a = O.Registration(factor=O.FACTOR_GICP, num_threads=0)
-        b = O.Registration(factor=O.FACTOR_GICP, num_threads=0, _lib=REF)
-        ra, rb = a.align(va, None, sc, np.eye(4)), b.align(vb, None, rsc, np.eye(4))
-        assert ra.iterations == rb.iterations and ra.num_inliers == rb.num_inliers
-        np.testing.assert_allclose(ra.T_target_source, rb.T_target_source, rtol=0, atol=1e-9)
+def test_voxelmap_and_vgicp_match(prepared, ref):
+    for offsets in R.OFFSETS:
+        out = R.voxelmap_outputs(None, prepared, offsets)
+        key = f"voxelmap/{offsets}"
+        same_digests({k: out[k] for k in (key + "/coords", key + "/counts", key + "/nn_idx", key + "/nn_found", "voxelmap/rows", key + "/query_rows")}, ref)
+        np.testing.assert_allclose(out["voxelmap/means"], ref["voxelmap/means"], rtol=0, atol=1e-12)
+        np.testing.assert_allclose(out["voxelmap/covs"], ref["voxelmap/covs"], rtol=0, atol=1e-12)
+        f = out[key + "/nn_found_sample"] == 1
+        np.testing.assert_allclose(out[key + "/nn_d2"][f], ref[key + "/nn_d2"][f], rtol=1e-12)
+        assert np.array_equal(out[key + "/align_stats"], ref[key + "/align_stats"])  # iterations, num_inliers
+        np.testing.assert_allclose(out[key + "/align_T"], ref[key + "/align_T"], rtol=0, atol=1e-9)
 
 
-def test_algebra_match():
-    rng = np.random.default_rng(1)
-    import ctypes as C
-
-    dp = C.POINTER(C.c_double)
-    for _ in range(10):
-        a = rng.normal(0, 0.5, 6)
-        T1 = O.se3_exp(a)
-        T2 = np.empty((4, 4))
-        REF.orc_se3_exp(a.ctypes.data_as(dp), T2.ctypes.data_as(dp))
-        np.testing.assert_allclose(T1, T2, rtol=0, atol=1e-15)
-        A = rng.normal(size=(6, 6))
-        A = A @ A.T + 1e-3 * np.eye(6)
-        bvec = rng.normal(size=6)
-        x2 = np.empty(6)
-        REF.orc_ldlt_solve6(A.ctypes.data_as(dp), bvec.ctypes.data_as(dp), x2.ctypes.data_as(dp))
+def test_algebra_match(ref):
+    for (a, A, bvec), T2, x2 in zip(R.algebra_inputs(), ref["algebra/se3_exp"], ref["algebra/ldlt_solve6"]):
+        np.testing.assert_allclose(O.se3_exp(a), T2, rtol=0, atol=1e-15)
         np.testing.assert_allclose(O.ldlt_solve6(A, bvec), x2, rtol=1e-12, atol=1e-14)
